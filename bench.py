@@ -104,7 +104,9 @@ def kernel_class_table(step_fn, ms_per_step):
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10,
+                    help="timed steps of every measurement of this path (headline, end-to-end, recipe and other "
+                         "configurations); the stock-PyTorch and CPU baselines time fixed short samples")
     ap.add_argument("--warmup", type=int, default=4)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--arch", default="ocrnet.HRNet_Mscale", choices=list(TFLOP_PER_CROP))
@@ -126,7 +128,14 @@ def parse():
                          "`vs_torch_gpu` to the line. Default at --gpus 1; this flag forces it for N > 1 (rank 0)")
     ap.add_argument("--no-torch-gpu-baseline", action="store_true")
     ap.add_argument("--no-recipe", action="store_true", help="skip the second (RMI + supervised multi-scale) measurement")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned to its caller as DIR/<name>.npy (float32): the loss, a "
+                         "fixed seeded sample of the gradients and of the updated parameters, the BatchNorm running "
+                         "statistics; the inputs depend on the arguments only, so two builds compare output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def peaks():
@@ -205,6 +214,27 @@ def workload_name(args):
     kind = "two-scale {0.5,1.0}" if args.arch in ("ocrnet.HRNet_Mscale", "mscale.HRNet") else "single-scale"
     return ("%s %s train step (zero_grad, fwd+bwd, SGD momentum + weight decay), %dx%d crops, "
             "%d crop/GPU, %s loss" % (args.arch, kind, args.height, args.width, args.batch_per_gpu, args.criterion.upper()))
+
+
+DUMP_SAMPLE = 4 * 1024 * 1024      # elements of each sampled array: 16 MB in float32
+
+
+def dump_outputs(out_dir, net, loss):
+    """--dump-outputs: the loss of the last step, the gradients it published into param.grad and the parameters the
+    optimizer left, both at the same DUMP_SAMPLE indices drawn from a fixed seed over the parameters in registration
+    order, and every BatchNorm running mean / variance."""
+    import numpy as np
+    params = [p for _, p in net.named_parameters()]
+    grads = torch.cat([p.grad.reshape(-1) for p in params])
+    values = torch.cat([p.detach().reshape(-1) for p in params])
+    g = torch.Generator().manual_seed(2024)
+    idx = torch.randint(0, grads.numel(), (min(DUMP_SAMPLE, grads.numel()),), generator=g).sort().values
+    idx = idx.to(grads.device)
+    running = torch.cat([b.reshape(-1).float() for n, b in net.named_buffers() if "running_" in n])
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (("loss", loss.detach().reshape(1)), ("grad_sample", grads[idx]), ("param_sample", values[idx]),
+                    ("bn_running_stats", running)):
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 def synth_batch(n, h, w, seed, device):
@@ -462,6 +492,8 @@ def run_b200(args):
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, net, loss)
     if os.environ.get("B200SEG_TIME_ONLY") == "1":              # A/B runs of a switch: the device-timed figure only
         if rank == 0:
             print(json.dumps(dict(ms_per_step=ms / args.steps, steps=args.steps, time_only=True)))
@@ -607,12 +639,12 @@ def run_b200(args):
             r0, r1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             torch.cuda.synchronize()
             r0.record()
-            for _ in range(10):
+            for _ in range(args.steps):
                 l2 = step2()
             r1.record()
             torch.cuda.synchronize()
-            ms2 = r0.elapsed_time(r1) / 10
-            line["train_recipe_rmi_sup"] = dict(value=B * 1000.0 / ms2, unit="crops/s", ms_per_step=ms2, steps=10,
+            ms2 = r0.elapsed_time(r1) / args.steps
+            line["train_recipe_rmi_sup"] = dict(value=B * 1000.0 / ms2, unit="crops/s", ms_per_step=ms2, steps=args.steps,
                                                 loss=float(l2), what="same step with criterion RMILoss and "
                                                 "supervised_mscale_loss_wt 0.05 (scripts/train_cityscapes.yml:21-24)")
             del net2, opt2
@@ -629,7 +661,7 @@ def run_b200(args):
             opt3 = _SGD3(net3.parameters(), lr=1e-3, momentum=0.9, weight_decay=1e-4)
             im2, gt2 = synth_batch(2, H, W, 7, "cpu")
             im2, gt2 = im2.cuda(), gt2.cuda()
-            for it in range(3 + 8):
+            for it in range(3 + args.steps):
                 if it == 3:
                     c0, c1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                     torch.cuda.synchronize()
@@ -640,7 +672,7 @@ def run_b200(args):
                 opt3.step()
             c1.record()
             torch.cuda.synchronize()
-            ms3 = c0.elapsed_time(c1) / 8
+            ms3 = c0.elapsed_time(c1) / args.steps
             extra["cfg2_ocrnet_HRNet_bs2_train"] = dict(
                 value=2 * 1000.0 / ms3, unit="crops/s", ms_per_step=ms3, tflops=2 * 7.77 / (ms3 * 1e-3),
                 what="ocrnet.HRNet single-scale train step, 2 x 1024x2048 crops per step, CE, bf16 storage / fp32 accumulate "
@@ -653,7 +685,7 @@ def run_b200(args):
             net4 = B200SegModule(args.arch, 19, n_scales=[0.5, 1.0, 2.0]).cuda().eval()
             from b200seg.evaltail import eval_minibatch
             with torch.no_grad():
-                for it in range(2 + 5):
+                for it in range(2 + args.steps):
                     if it == 2:
                         c0, c1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                         torch.cuda.synchronize()
@@ -661,7 +693,7 @@ def run_b200(args):
                     res = eval_minibatch(net4, images_d, gts_d, scales=(1.0,), do_flip=False)
                 c1.record()
                 torch.cuda.synchronize()
-            ms4 = c0.elapsed_time(c1) / 5
+            ms4 = c0.elapsed_time(c1) / args.steps
             extra["cfg5_three_scale_inference"] = dict(
                 value=1000.0 / ms4, unit="frames/s", ms_per_frame=ms4, tflops=16.04 / (ms4 * 1e-3),
                 what="ocrnet.HRNet_Mscale nscale_forward {0.5,1.0,2.0} on a 1024x2048 frame + device-side argmax / "
@@ -674,7 +706,7 @@ def run_b200(args):
             net5 = B200SegModule("deepv3.DeepV3PlusW38", 19, criterion="ce", use_cuda_graph=not args.no_graph).cuda().train()
             from b200seg.optim import FusedSGD as _SGD5
             opt5 = _SGD5(net5.parameters(), lr=1e-3, momentum=0.9, weight_decay=1e-4)
-            for it in range(3 + 6):
+            for it in range(3 + args.steps):
                 if it == 3:
                     c0, c1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                     torch.cuda.synchronize()
@@ -685,7 +717,7 @@ def run_b200(args):
                 opt5.step()
             c1.record()
             torch.cuda.synchronize()
-            ms5 = c0.elapsed_time(c1) / 6
+            ms5 = c0.elapsed_time(c1) / args.steps
             extra["cfg4_deepv3_w38_train"] = dict(
                 value=1000.0 / ms5, unit="crops/s", ms_per_step=ms5, tflops=34.95 / (ms5 * 1e-3), loss=float(l5),
                 what="deepv3.DeepV3PlusW38 train step (WRN-38 trunk at output stride 8, dilations 2/4, ASPP 12/24/36, "

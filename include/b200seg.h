@@ -349,8 +349,11 @@ int b200seg_transpose_pad(const void* src, int32_t src_fp32, int32_t R, int32_t 
 int b200seg_cast_rows(const float* src, int32_t src_ld, void* dst_bf16, int32_t dst_ld, int64_t rows, int32_t C,
                       int32_t accumulate, void* stream);
 
-/* db[c] += sum_rows dy[row][c], c < C <= 32 (bias gradient of the logit heads, network/ocrnet.py:66-76) */
-int b200seg_bias_grad(const void* dy_bf16, int32_t ld, int64_t rows, int32_t C, float* db, void* stream);
+/* db[c] += sum_rows dy[row][c], c < C <= 32 (bias gradient of the logit heads, network/ocrnet.py:66-76). partials is an
+ * fp32 workspace of b200seg_bias_grad_blocks(rows) * 32 floats: the per-block sums are added in a fixed order (no
+ * atomics), so the result does not depend on the order in which blocks finish. Two launches. */
+int32_t b200seg_bias_grad_blocks(int64_t rows);
+int b200seg_bias_grad(const void* dy_bf16, int32_t ld, int64_t rows, int32_t C, float* partials, float* db, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Multi-scale attention blend + cross-entropy, forward and backward (network/ocrnet.py:170-183,264-319,

@@ -136,7 +136,8 @@ SIGNATURES = {
     "b200seg_class_softmax_bwd": (ctypes.c_int, [V, I32, V, I64, I32, F, V, V]),
     "b200seg_transpose_pad": (ctypes.c_int, [V, I32, I32, I32, I32, V, I32, V]),
     "b200seg_cast_rows": (ctypes.c_int, [V, I32, V, I32, I64, I32, I32, V]),
-    "b200seg_bias_grad": (ctypes.c_int, [V, I32, I64, I32, V, V]),
+    "b200seg_bias_grad_blocks": (I32, [I64]),
+    "b200seg_bias_grad": (ctypes.c_int, [V, I32, I64, I32, V, V, V]),
     "b200seg_count_valid": (ctypes.c_int, [V, I64, I32, I32, V, V, V]),
     "b200seg_rmi_pool": (ctypes.c_int, [ctypes.POINTER(MscaleDesc), V, V, V, V, V, V]),
     "b200seg_rmi_ws_bytes": (c_size_t, [I32]),

@@ -503,7 +503,9 @@ def cast_rows(src, dst, C, accumulate=False):
 
 def bias_grad(dy, C, db):
     rows = dy.numel() // dy.shape[-1]
-    check(lib().b200seg_bias_grad(ptr(dy), _ld(dy), rows, C, ptr(db), stream_ptr()), "bias_grad")
+    L = lib()
+    partials = _new(L.b200seg_bias_grad_blocks(rows) * 32, dtype=F32, device=dy.device)
+    check(L.b200seg_bias_grad(ptr(dy), _ld(dy), rows, C, ptr(partials), ptr(db), stream_ptr()), "bias_grad", launches=2)
 
 
 # ----------------------------------------------------------------------------------------------- mscale + loss

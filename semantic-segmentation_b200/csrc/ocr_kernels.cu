@@ -272,9 +272,11 @@ __global__ void cast_rows_kernel(const float* __restrict__ src, int src_ld, __nv
 }
 
 
-// db[c] += sum_rows dy[row][c]  for c < C  (conv bias gradient of the logit heads; dy bf16 [rows][ld])
+// partials[block][c] = sum over the block's rows of dy[row][c] for c < C (conv bias gradient of the logit heads; dy bf16
+// [rows][ld]). The blocks' sums are combined by colsum_finish_kernel in a fixed order, not with atomics, so the gradient
+// is the same bit for bit on every run.
 __global__ void __launch_bounds__(256)
-colsum_kernel(const __nv_bfloat16* __restrict__ dy, int ld, long long rows, int C, float* __restrict__ db) {
+colsum_kernel(const __nv_bfloat16* __restrict__ dy, int ld, long long rows, int C, float* __restrict__ partials) {
   pdl_sync();
   // thread (r, c): 8 row-lanes x 32 columns
   const int c = threadIdx.x & 31, r = threadIdx.x >> 5;
@@ -285,10 +287,27 @@ colsum_kernel(const __nv_bfloat16* __restrict__ dy, int ld, long long rows, int 
   __shared__ float s[8][32];
   s[r][c] = acc;
   __syncthreads();
+  if (r == 0) {
+    float t = 0.f;
+    for (int i = 0; i < 8; ++i) t += s[i][c];
+    partials[blockIdx.x * 32 + c] = t;
+  }
+}
+
+// db[c] += sum over blocks of partials[block][c], always in the same order
+__global__ void __launch_bounds__(256)
+colsum_finish_kernel(const float* __restrict__ partials, int nblocks, int C, float* __restrict__ db) {
+  pdl_sync();
+  const int c = threadIdx.x & 31, r = threadIdx.x >> 5;
+  float acc = 0.f;
+  for (int b = r; b < nblocks; b += 8) acc += partials[b * 32 + c];
+  __shared__ float s[8][32];
+  s[r][c] = acc;
+  __syncthreads();
   if (r == 0 && c < C) {
     float t = 0.f;
     for (int i = 0; i < 8; ++i) t += s[i][c];
-    atomicAdd(db + c, t);
+    db[c] += t;
   }
 }
 
@@ -366,11 +385,17 @@ extern "C" int b200seg_cast_rows(const float* src, int32_t src_ld, void* dst_bf1
   RET_LAUNCH();
 }
 
-extern "C" int b200seg_bias_grad(const void* dy_bf16, int32_t ld, int64_t rows, int32_t C, float* db, void* stream) {
-  if (!dy_bf16 || !db || C > 32) return B200SEG_E_BADARG;
-  long long b = (rows + 7) / 8;
-  if (b > 148 * 4) b = 148 * 4;
-  launch_k(colsum_kernel, dim3((int)b), dim3(256), 0, (cudaStream_t)stream, (const __nv_bfloat16*)dy_bf16, ld, rows,
-           C, db);
+extern "C" int32_t b200seg_bias_grad_blocks(int64_t rows) {
+  const long long b = (rows + 7) / 8;
+  return (int32_t)(b < 1 ? 1 : (b > 148 * 4 ? 148 * 4 : b));
+}
+
+extern "C" int b200seg_bias_grad(const void* dy_bf16, int32_t ld, int64_t rows, int32_t C, float* partials, float* db,
+                                 void* stream) {
+  if (!dy_bf16 || !partials || !db || C > 32) return B200SEG_E_BADARG;
+  const int b = b200seg_bias_grad_blocks(rows);
+  launch_k(colsum_kernel, dim3(b), dim3(256), 0, (cudaStream_t)stream, (const __nv_bfloat16*)dy_bf16, ld, rows,
+           C, partials);
+  launch_k(colsum_finish_kernel, dim3(1), dim3(256), 0, (cudaStream_t)stream, (const float*)partials, b, C, db);
   RET_LAUNCH();
 }

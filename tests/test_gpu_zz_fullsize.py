@@ -226,3 +226,47 @@ def test_w48_step_against_the_committed_reference_vectors(golden):
     # measured: attention 0.12, prediction 0.74 (dominated by the saturated soft-region softmax of these weights; the
     # well-conditioned eval comparison is test_full_size_value_parity_vs_gpu_oracle: 1.3 % / 99.99 % argmax)
     assert r_attn <= 0.3 and r_pred <= 1.0, (r_pred, r_attn)
+
+
+def _seeded_training_run(steps):
+    from b200seg.module import B200SegModule
+    from b200seg.optim import FusedSGD
+    torch.manual_seed(0)
+    net = B200SegModule("ocrnet.HRNet_Mscale", 19).cuda().train()
+    with torch.no_grad():
+        for n_, p_ in net.named_parameters():
+            if p_.dim() == 4 and n_.startswith("backbone"):
+                p_.normal_(0, (2.0 / (p_.shape[1] * p_.shape[2] * p_.shape[3])) ** 0.5)
+    opt = FusedSGD(net.parameters(), lr=1e-3, momentum=0.9, weight_decay=1e-4)
+    g = torch.Generator().manual_seed(1)
+    images = torch.randn((1, 3, 1024, 2048), generator=g).cuda()
+    gts = torch.randint(0, 19, (1, 1024, 2048), generator=g)
+    gts[:, :8] = 255
+    gts = gts.cuda()
+    losses = []
+    for _ in range(steps):                     # eager warm-up, capture, replays; Dropout2d on, masks from the seed
+        opt.zero_grad(set_to_none=True)
+        loss = net({"images": images, "gts": gts})
+        loss.backward()
+        opt.step()
+        losses.append(loss.detach().clone())
+    torch.cuda.synchronize()
+    out = dict(loss=torch.stack(losses).cpu(),
+               grad=torch.cat([p.grad.reshape(-1) for p in net.parameters()]).cpu(),
+               param=torch.cat([p.detach().reshape(-1) for p in net.parameters()]).cpu(),
+               running=torch.cat([b.reshape(-1).float() for n, b in net.named_buffers() if "running_" in n]).cpu())
+    del net, opt
+    torch.cuda.empty_cache()
+    return out
+
+
+@pytest.mark.timeout(600)
+def test_seeded_full_size_training_is_bit_identical():
+    """bench.py's training loop (two-scale 1024x2048 step, Dropout2d on, FusedSGD) run twice from the same seed gives the
+    same losses, gradients, parameters and BatchNorm running statistics bit for bit: no reduction of the step depends on
+    the order in which blocks or streams finish. Otherwise a one-ulp difference grows over a few steps of training into
+    different gradients, and two runs of the benchmark cannot be compared output for output."""
+    a, b = _seeded_training_run(5), _seeded_training_run(5)
+    for k in a:
+        diff = int((a[k] != b[k]).sum())
+        assert diff == 0, (k, diff, float((a[k] - b[k]).abs().max()))
